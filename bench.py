@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (libkivi_b200 fused decode)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU fake-quant path
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's logits / ids as .npy
 
 Metric (BASELINE.json): decode tokens/sec @ Llama-2-7B bs32 seq4k K2V2 g32 R128.  A "step" is one decode step of the
 whole model for the batch: 32 x [RMSNorm, q/k/v proj, RoPE, KIVI decode attention + cache update (two libkivi_b200
@@ -256,8 +257,9 @@ def attention_roofline(model, cache, step_ms):
     return roof
 
 
-def run_decode(model_name, B, seq, K, W, rank, ws, local, sampler=None, e2e=True, kivi=None, roofline=True):
-    """Build the model, pre-fill the cache so that the K timed steps end at kv length `seq`, time K graph-replayed steps."""
+def run_decode(model_name, B, seq, K, W, rank, ws, local, sampler=None, e2e=True, kivi=None, roofline=True, keep_outputs=False):
+    """Build the model, pre-fill the cache so that the K timed steps end at kv length `seq`, time K graph-replayed steps.
+    keep_outputs: res["outputs"] holds, as numpy arrays, what the last timed step returned to its caller."""
     import torch
     from kivi_b200 import dist as kdist
     from kivi_b200.llama_kivi import LlamaForCausalLM_KIVI, default_config
@@ -346,6 +348,8 @@ def run_decode(model_name, B, seq, K, W, rank, ws, local, sampler=None, e2e=True
            "clocks": sampler.window(t_host0, t_host1) if sampler is not None else None}
     all_ids = model.all_tokens
     assert all_ids.numel() == Bg
+    if keep_outputs:                                         # read before the e2e steps overwrite the static buffers
+        res["outputs"] = {"logits": model._logits.cpu().numpy(), "next_tokens": all_ids.cpu().numpy()}
     if ws > 1:                                               # the general path, for the record: full-logits all-gather
         torch.cuda.synchronize()
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -474,6 +478,26 @@ def reference_gpu_timing(B, H, Hkv, T, bits, g, R):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Write what the last timed step returned as <out_dir>/<name>.npy, so that two builds can be compared output for
+    output: logits.npy (fp32 [rows, vocab], this rank's sequences), logits_rows.npy (the sequences those rows belong to)
+    and next_tokens.npy (the sampled ids of every rank, as float64: exact).  When all of this rank's logits would exceed
+    DUMP_LIMIT_BYTES, a fixed sample of its sequences (seed 0) is written instead."""
+    import numpy as np
+    logits, tokens = outputs["logits"], outputs["next_tokens"].astype(np.float64)
+    rows = np.arange(logits.shape[0])
+    cap = (DUMP_LIMIT_BYTES - 3 * 4096 - tokens.nbytes - logits.shape[0] * 8) // (logits.shape[1] * 4)   # 3 npy headers
+    if rows.size > cap:
+        rows = np.sort(np.random.default_rng(0).choice(rows.size, cap, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), np.ascontiguousarray(logits[rows], np.float32))
+    np.save(os.path.join(out_dir, "logits_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "next_tokens.npy"), tokens)
+
+
 # --------------------------------------------------------------------------------------------------
 # main arm
 # --------------------------------------------------------------------------------------------------
@@ -493,9 +517,12 @@ def run_ours(args):
         sampler.start()
     B = args.batch if args.global_batch is None else args.global_batch // ws
     kivi = dict(k_bits=args.k_bits, v_bits=args.v_bits, group_size=args.group_size, residual_length=args.residual_length)
-    main = run_decode(args.model, B, args.seq, K, W, rank, ws, local, sampler=sampler, kivi=kivi)
+    main = run_decode(args.model, B, args.seq, K, W, rank, ws, local, sampler=sampler, kivi=kivi,
+                      keep_outputs=args.dump_outputs is not None)
     if main is None:
         return 0
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, main.pop("outputs"))
     model = main.pop("model")
     mcfg = model.config
     roof = main.get("roofline")
@@ -608,8 +635,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-reference-gpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra BASELINE configs (cfg 3 / 4 / 5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (logits, sampled ids) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs is not None:
+            ap.error("--dump-outputs applies to the default --impl ours")
         return run_reference(args)
     return run_ours(args)
 

@@ -70,10 +70,10 @@ def gen_pack_tensor():
 
 
 def gen_fake_quant():
-    """cfg 1 shape family: [1,H,256,128] K2V2 g32 (reduced H to keep the fixture small)."""
+    """cfg 1 shape family: [1,H,256,128] K2V2 g32 (H = 2 keeps the fixture under 1 MB)."""
     out = {}
     torch.manual_seed(11)
-    B, H, T, D, g = 1, 4, 256, 128, 32
+    B, H, T, D, g = 1, 2, 256, 128, 32
     for bits in (2, 4):
         k = torch.randn(B, H, T, D, dtype=torch.float16)
         v = torch.randn(B, H, T, D, dtype=torch.float16)

@@ -1,11 +1,14 @@
 """Parity of the CUDA dequant-GEMVs (kivi_bgemv.cu through the C ABI / Python surface) with the oracle
-(reference summation order, oracle/kivi_oracle.c) and -- when oracle/_ref/kivi_gemv.so is present --
-with the UNMODIFIED reference CUDA extension on the same inputs.  Tolerance: tests/_util.py."""
+(reference summation order, oracle/kivi_oracle.c) and with the stored outputs of the UNMODIFIED reference CUDA
+extension on the same inputs.  Tolerance: tests/_util.py."""
+import hashlib
+import os
+
 import numpy as np
 import pytest
 import torch
 
-from oracle import build_ref, ref
+from oracle import ref
 from tests._util import assert_gemv_close, l1_mass_ref_layout, to_np
 
 pytestmark = pytest.mark.gpu
@@ -136,27 +139,35 @@ def test_kernel_layout_reference_test_case(BIT, mqa):
     assert mean_rel < 1e-4
 
 
-@pytest.mark.parametrize("BIT", [2, 4])
-def test_against_reference_cuda_extension(BIT):
-    """Kernel-vs-kernel (the only place the 1e-3 rtol bar is meaningful, SURVEY section 4): our library
-    and the oracle against the UNMODIFIED reference extension compiled for sm_100a (oracle/_ref)."""
-    refmod = build_ref.load()
-    if refmod is None:
-        pytest.skip("oracle/_ref/kivi_gemv.so not built (needs /root/reference at build time)")
-    from kivi_b200 import kivi_gemv, matmul
+REFERENCE_EXT_GOLDEN = "gemv_ext_reference.npz"
+
+
+def reference_ext_cases(BIT):
+    """Seeded inputs of test_against_reference_cuda_extension, case by case: (case key, (B, nh, nh_kv, IC, OC, GS),
+    inp, code / scale / mn in the reference layout, the same transposed to the kernel layout, sha256 of the kernel
+    inputs).  tests/golden/make_golden_ext.py runs the reference extension on exactly these."""
     rng = np.random.default_rng(1)
-    for (B, nh, nh_kv, IC, OC, GS) in [(2, 8, 8, 739, 128, 32), (2, 8, 2, 128, 1024, 32), (1, 4, 1, 333, 128, 64)]:
+    for i, (B, nh, nh_kv, IC, OC, GS) in enumerate([(2, 8, 8, 739, 128, 32), (2, 8, 2, 128, 1024, 32), (1, 4, 1, 333, 128, 64)]):
         nkv = B * nh_kv
         inp = rng.standard_normal((B * nh, 1, IC)).astype(np.float16)
         w = rng.standard_normal((nkv, IC, OC)).astype(np.float16)
         code, scale, mn = ref.pack_lastdim(w, GS, BIT)
-        qw_t = np.ascontiguousarray(code.transpose(0, 2, 1))
-        sc_t = np.ascontiguousarray(scale.transpose(0, 2, 1))
-        mn_t = np.ascontiguousarray(mn.transpose(0, 2, 1))
+        kernel_layout = [np.ascontiguousarray(a.transpose(0, 2, 1)) for a in (code, scale, mn)]
+        digest = hashlib.sha256(b"".join(a.tobytes() for a in [inp] + kernel_layout)).hexdigest()
+        yield f"bit{BIT}_case{i}", (B, nh, nh_kv, IC, OC, GS), inp, (code, scale, mn), kernel_layout, digest
+
+
+@pytest.mark.parametrize("BIT", [2, 4])
+def test_against_reference_cuda_extension(golden_dir, BIT):
+    """Kernel-vs-kernel (the only place the 1e-3 rtol bar is meaningful, SURVEY section 4): our library
+    and the oracle against the outputs of the UNMODIFIED reference extension compiled for sm_100a and run on a B200
+    (tests/golden/gemv_ext_reference.npz, made by tests/golden/make_golden_ext.py on the same seeded inputs)."""
+    from kivi_b200 import kivi_gemv, matmul
+    gold = np.load(os.path.join(golden_dir, REFERENCE_EXT_GOLDEN))
+    for key, (B, nh, nh_kv, IC, OC, GS), inp, (code, scale, mn), (qw_t, sc_t, mn_t), digest in reference_ext_cases(BIT):
+        assert str(gold[key + "_inputs_sha256"]) == digest, f"{key}: inputs differ from those the golden outputs were made from"
+        ref_out = gold[key + "_out"]
         args = [torch.from_numpy(a).cuda() for a in (inp, qw_t, sc_t, mn_t)]
-        ref_out = refmod.gemv_forward_cuda_outer_dim(*args, BIT, GS, nh, nh_kv)
-        torch.cuda.synchronize()
-        ref_out = to_np(ref_out)
         # (1) the C oracle reproduces the reference kernel BIT FOR BIT (same order, fmaf contraction)
         orc = ref.bgemv_outer_kernel_layout(inp, qw_t, sc_t, mn_t, BIT, GS, nh, nh_kv)
         np.testing.assert_array_equal(orc.view(np.uint16), ref_out.view(np.uint16))
