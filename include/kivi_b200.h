@@ -262,6 +262,35 @@ int kivi_silu_mul_f16(const void* gate_up, void* out, int rows, int intermediate
 int kivi_greedy_sample_exchange_f32(const void* logits, int batch, int vocab, void* next_local, void* ids_feedback,
                                     const void* peer_buffers, int rank, int world, const void* step, void* err, void* stream);
 
+/* Sampled decoding fused with the same exchange (temperature -> top-k -> top-p -> one draw; the order and definitions of
+ * transformers' TemperatureLogitsWarper, TopKLogitsWarper, TopPLogitsWarper).  Per row b of logits fp32 [batch, vocab], with
+ * T = temperature[b], k = top_k[b], p = top_p[b]:
+ *   1. x_v = fp32(l_v / T) (IEEE division, as `scores / temperature`).  T <= 0: a GREEDY row, the argmax with the rule of
+ *      kivi_greedy_sample_exchange_f32 (greedy and sampled rows may share a batch).  For sampled rows a NaN x counts as -inf.
+ *   2. top-k (off when k <= 0 or k >= vocab): keep x_v >= x_(k), the k-th largest value; all ties at the threshold stay.
+ *   3. top-p (off when p >= 1) over the top-k survivors, with e_v = exp(x_v - max x) and Z1 = sum e: keep v iff S_>(v) < p*Z1,
+ *      S_>(v) = mass of the survivors with a strictly larger x (HF: drop where the ascending cumulative mass <= 1 - p;
+ *      restated without a sort, so ties share one fate).  The maximum is always kept.
+ *   4. draw: u = ((r0 >> 8) + 0.5) * 2^-24, r0 = word 0 of Philox4x32-10 with key (seed lo, seed hi) and counter
+ *      (counter lo, counter hi, row_offset + b, 0).  The id is the smallest kept v (index order) whose running sum of e over
+ *      the kept tokens exceeds u * Z_K, Z_K = the total of that sum; the last kept token if none does.
+ * The masses are summed in 2^-40 fixed point, so every sum is exact and order-free: the ids are a pure function of (seed,
+ * counter, row_offset + b, the logits row) -- the same in eager and graph mode, for any batch split across ranks, and from
+ * run to run.  A row holding NaN or +-inf still yields an id in [0, vocab) (at an infinite maximum the tokens equal to it
+ * share the mass).  vocab <= 262144; one cluster of up to 8 CTAs per row, the row held in shared memory.
+ * next_local / ids_feedback / peer_buffers / rank / world / step / err: exactly as kivi_greedy_sample_exchange_f32. */
+typedef struct kivi_sampling {
+    const float*    temperature;  /* device [batch]; <= 0: greedy row                       */
+    const int32_t*  top_k;        /* device [batch]; <= 0 or >= vocab: off                  */
+    const float*    top_p;        /* device [batch]; >= 1: off                              */
+    const uint64_t* seed;         /* device, 1 word                                         */
+    const int64_t*  counter;      /* device, 1 word; the caller increments it before a call */
+    int32_t         row_offset;   /* global index of row 0 (rank * batch)                   */
+} kivi_sampling_t;
+int kivi_sample_exchange_f32(const void* logits, int batch, int vocab, const kivi_sampling_t* s,
+                             void* next_local, void* ids_feedback, const void* peer_buffers,
+                             int rank, int world, const void* step, void* err, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

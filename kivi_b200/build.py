@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(CSRC, "libkivi_b200.so")
 SOURCES = ["kivi_api.cu", "kivi_pack.cu", "kivi_bgemv.cu", "kivi_bgemv_mma.cu", "kivi_cache.cu", "kivi_decode.cu", "kivi_attn_k2v2.cu",
-           "kivi_attn_k4v4.cu", "kivi_attn_k2v4.cu", "kivi_attn_k4v2.cu", "kivi_model.cu"]
+           "kivi_attn_k4v4.cu", "kivi_attn_k2v4.cu", "kivi_attn_k4v2.cu", "kivi_model.cu", "kivi_sample.cu"]
 HEADERS = ["kivi_common.cuh", "kivi_decode.cuh", "kivi_attn.cuh", os.path.join("..", "..", "include", "kivi_b200.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]

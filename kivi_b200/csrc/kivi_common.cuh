@@ -123,4 +123,65 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Token sampling + exchange, shared by the greedy (kivi_model.cu) and the sampling (kivi_sample.cu) kernels.
+// ---------------------------------------------------------------------------------------------
+// The argmax order of torch.argmax: a NaN beats every number, and among NaNs, as among equal maxima, the lower index wins.
+// It is a total order, so every reduction tree over (value, index) pairs ends at the same pair.
+__device__ __forceinline__ bool argmax_takes(float best, int bi, float ov, int oi) {
+    return (ov != ov) ? (!(best != best) || oi < bi) : (!(best != best) && (ov > best || (ov == best && oi < bi)));
+}
+
+__device__ __forceinline__ void warp_argmax(float& best, int& bi) {
+    #pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (argmax_takes(best, bi, ov, oi)) { best = ov; bi = oi; }
+    }
+}
+
+// The ids of one step travel to every data-parallel replica (kivi_greedy_sample_exchange_f32 in include/kivi_b200.h):
+//   peer[p]  : rank p's buffer: int64 tokens[2][world * B] (double-buffered by step parity), then uint64 arrived[world]
+//   step     : device counter, incremented by the caller BEFORE the launch (inside the same CUDA graph)
+// peer == nullptr: one GPU, no exchange.
+struct TokenExchange {
+    long long* const* peer;
+    int B, rank, world;
+    const int* step;
+    int* err;
+};
+
+// One thread per sequence: the id of sequence b goes to next_local, ids_feedback (may be NULL) and -- replicas -- into this
+// rank's slot of EVERY rank's token buffer with plain peer stores over NVLink / NVSwitch, then releases a per-rank arrival
+// counter on every peer.
+__device__ __forceinline__ void exchange_publish(long long tok, int b, long long* next_local, long long* ids_feedback,
+                                                 const TokenExchange& x) {
+    next_local[b] = tok;
+    if (ids_feedback) ids_feedback[b] = tok;
+    if (x.peer) {
+        const int step = *x.step;
+        const long long slot = (long long)(step & 1) * x.world * x.B + (long long)x.rank * x.B + b;
+        for (int p = 0; p < x.world; ++p) x.peer[p][slot] = tok;
+        __threadfence_system();                                             // the ids are visible system-wide before the arrivals
+        for (int p = 0; p < x.world; ++p)
+            atomicAdd_system(reinterpret_cast<unsigned long long*>(x.peer[p] + 2ll * x.world * x.B + x.rank), 1ull);
+    }
+}
+
+// Threads tid < world of ONE block wait (bounded) until all ranks' ids of this step have arrived in this rank's buffer; on
+// time-out *err = 1 instead of hanging the GPU.
+__device__ __forceinline__ void exchange_wait(const TokenExchange& x, int tid) {
+    if (!x.peer || tid >= x.world) return;
+    const unsigned long long want = (unsigned long long)(*x.step) * (unsigned long long)x.B;
+    const volatile unsigned long long* cnt =
+        reinterpret_cast<const volatile unsigned long long*>(x.peer[x.rank] + 2ll * x.world * x.B + tid);
+    long long spins = 0;
+    while (*cnt < want) {
+        if (++spins > (1ll << 24)) { *x.err = 1; break; }                  // ~ a second: a peer is gone
+        __nanosleep(64);
+    }
+    __threadfence_system();
+}
+
 }  // namespace kivi

@@ -112,9 +112,8 @@ silu_mul_kernel(const __half* __restrict__ gu, __half* __restrict__ out, int I)
 // to peer memory over NVLink / NVSwitch (the buffers are one symmetric allocation, torch.distributed._symmetric_memory) --
 // and releases a per-rank arrival counter on every peer.  Block 0 then waits (bounded) until all ranks' ids of this step have
 // arrived here.  Argmax is local to a sequence, so the data-parallel replicas exchange 8 bytes per sequence and nothing of
-// the next step depends on the exchange: no rank ever blocks another one's critical path.
-//   peer[p]  : rank p's buffer: int64 tokens[2][world * B] (double-buffered by step parity), then uint64 arrived[world]
-//   step     : device counter, incremented by the caller BEFORE the launch (inside the same CUDA graph)
+// the next step depends on the exchange: no rank ever blocks another one's critical path.  The buffer layout, the stores
+// and the bounded wait are exchange_publish / exchange_wait (kivi_common.cuh), shared with the sampling kernel.
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 greedy_exchange_kernel(const float* __restrict__ logits, int V, long long* __restrict__ next_local, long long* __restrict__ ids_feedback,
@@ -123,51 +122,23 @@ greedy_exchange_kernel(const float* __restrict__ logits, int V, long long* __res
     __shared__ float smax[8];
     __shared__ int sidx[8];
     const int b = blockIdx.x, tid = threadIdx.x;
+    const TokenExchange x{peer, B, rank, world, step_ptr, err};
     const float* row = logits + (long long)b * V;
     float best = -INFINITY;
     int bi = 0x7fffffff;
     for (int i = tid; i < V; i += 256) {
         const float v = row[i];
-        if (v > best || (v == best && i < bi) || (v != v && !(best != best))) { best = v; bi = i; }   // a NaN wins, like torch.argmax
+        if (argmax_takes(best, bi, v, i)) { best = v; bi = i; }             // a NaN wins, like torch.argmax
     }
-    #pragma unroll
-    for (int o = 16; o >= 1; o >>= 1) {
-        const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-        const bool take = (ov != ov) ? (!(best != best) || oi < bi) : (!(best != best) && (ov > best || (ov == best && oi < bi)));
-        if (take) { best = ov; bi = oi; }
-    }
+    warp_argmax(best, bi);
     if ((tid & 31) == 0) { smax[tid >> 5] = best; sidx[tid >> 5] = bi; }
     __syncthreads();
     if (tid == 0) {
-        for (int w = 1; w < 8; ++w) {
-            const float ov = smax[w];
-            const int oi = sidx[w];
-            const bool take = (ov != ov) ? (!(best != best) || oi < bi) : (!(best != best) && (ov > best || (ov == best && oi < bi)));
-            if (take) { best = ov; bi = oi; }
-        }
-        const long long tok = bi;
-        next_local[b] = tok;
-        if (ids_feedback) ids_feedback[b] = tok;
-        if (peer) {
-            const int step = *step_ptr;
-            const long long slot = (long long)(step & 1) * world * B + (long long)rank * B + b;
-            for (int p = 0; p < world; ++p) peer[p][slot] = tok;
-            __threadfence_system();                                         // the ids are visible system-wide before the arrivals
-            for (int p = 0; p < world; ++p)
-                atomicAdd_system(reinterpret_cast<unsigned long long*>(peer[p] + 2ll * world * B + rank), 1ull);
-        }
+        for (int w = 1; w < 8; ++w)
+            if (argmax_takes(best, bi, smax[w], sidx[w])) { best = smax[w]; bi = sidx[w]; }
+        exchange_publish(bi, b, next_local, ids_feedback, x);
     }
-    if (peer && b == 0 && tid < world) {                                     // all ranks' ids of this step are here before the kernel ends
-        const unsigned long long want = (unsigned long long)(*step_ptr) * (unsigned long long)B;
-        const volatile unsigned long long* cnt = reinterpret_cast<const volatile unsigned long long*>(peer[rank] + 2ll * world * B + tid);
-        long long spins = 0;
-        while (*cnt < want) {
-            if (++spins > (1ll << 24)) { *err = 1; break; }                  // ~ a second: a peer is gone; report instead of hanging the GPU
-            __nanosleep(64);
-        }
-        __threadfence_system();
-    }
+    if (b == 0) exchange_wait(x, tid);                                       // all ranks' ids of this step are here before the kernel ends
 }
 
 }  // namespace kivi

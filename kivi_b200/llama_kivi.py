@@ -348,6 +348,9 @@ class LlamaForCausalLM_KIVI(nn.Module):
         self._dist_tokens = None            # [world * B] ids gathered inside the step (greedy sampling, world > 1)
         self._dist_in_graph = True
         self._exchange = None               # kivi_b200.dist.PeerTokenExchange: ids stored into the peers' buffers by the sampling kernel
+        self._sampling_user = None          # the values given to set_sampling (generate's base values)
+        self._sampling_cfg = None           # the values decode_step samples with (None: greedy decoding)
+        self._sampling = None               # glue.SamplingParams: their device buffers, sized to the cache's batch
 
     # ------------------------------------------------------------------ HF-style construction
     @classmethod
@@ -545,7 +548,8 @@ class LlamaForCausalLM_KIVI(nn.Module):
         self._pos = torch.zeros((batch, 1), dtype=torch.long, device=dev)
         self._ids = torch.zeros((batch, 1), dtype=torch.long, device=dev)
         self._logits = torch.zeros((batch, cfg.vocab_size), dtype=torch.float32, device=dev)
-        self.next_tokens = torch.zeros((batch,), dtype=torch.long, device=dev)   # greedy argmax of the step (in-graph)
+        self.next_tokens = torch.zeros((batch,), dtype=torch.long, device=dev)   # the ids sampled by the step (in-graph)
+        self._sampling = None
         self._tables(dev)                                    # rows for every position the cache can reach
         return self.cache
 
@@ -593,14 +597,19 @@ class LlamaForCausalLM_KIVI(nn.Module):
             self._logits.copy_(self.lm_head(h[:, 0]).float())
         self.cache_advance_device()
         self._pos.add_(1)
-        # greedy sampling inside the step (and inside its CUDA graph): the argmax of a sequence needs only that
-        # sequence's logits, so with data-parallel replicas the exchange is the sampled ids, 8 B per sequence
+        # sampling inside the step (and inside its CUDA graph): the id of a sequence needs only that sequence's logits,
+        # so with data-parallel replicas the exchange is the sampled ids, 8 B per sequence
         from . import glue
         if self._exchange is not None:
             self._exchange.step.add_(1)                      # the step number the peers' arrival counters are compared with
-        # one kernel: argmax per sequence, the feed-back copy for the next step, and (replicas) the ids stored straight into
-        # every peer's buffer over NVLink + arrival counters
-        glue.greedy_sample(self._logits, self.next_tokens, self._ids.view(-1), self._exchange)
+        # one kernel: argmax (or temperature / top-k / top-p draw) per sequence, the feed-back copy for the next step, and
+        # (replicas) the ids stored straight into every peer's buffer over NVLink + arrival counters
+        if self._sampling_cfg is None:
+            glue.greedy_sample(self._logits, self.next_tokens, self._ids.view(-1), self._exchange)
+        else:
+            sp = self._sampling_params()
+            sp.counter.add_(1)                               # a new uniform per step, also on graph replays
+            glue.sample(self._logits, sp, self.next_tokens, self._ids.view(-1), self._exchange)
         if self._dist_tokens is not None and self._dist_in_graph:
             from . import dist as kdist
             kdist.gather_tokens(self.next_tokens, out=self._dist_tokens)
@@ -618,6 +627,43 @@ class LlamaForCausalLM_KIVI(nn.Module):
             self._dist_tokens = torch.zeros(world_size * self.cache.batch, dtype=torch.long, device=self.cache.device)
         self._dist_in_graph = in_graph
         self._graph = None
+
+    def set_sampling(self, temperature=1.0, top_k=0, top_p=1.0, seed: int | None = None):
+        """Sample the steps of decode_step with temperature -> top-k -> top-p (transformers' warpers; kivi_sample_exchange_f32
+        in include/kivi_b200.h); `set_sampling(None)` returns to greedy decoding.  Every value is one number or one per
+        sequence: temperature 0 makes that sequence greedy, top_k 0 and top_p 1 switch the filter off.  seed=None draws one
+        from torch's default generator (torch.manual_seed makes it reproducible).  Changing values is a device copy that
+        the captured step sees; switching between greedy and sampling re-captures the step.  The draw counter restarts at 0."""
+        self._sampling_user = None if temperature is None else dict(temperature=temperature, top_k=top_k, top_p=top_p,
+                                                                       seed=seed)
+        self._activate_sampling(self._sampling_user)
+
+    def _activate_sampling(self, cfg):
+        if cfg is None:
+            if self._sampling_cfg is not None:
+                self._graph = None
+            self._sampling_cfg = None
+            return
+        cfg = dict(cfg)
+        if cfg["seed"] is None:
+            cfg["seed"] = int(torch.randint(0, 2 ** 63 - 1, (1,)).item())
+        if self._sampling_cfg is None:
+            self._graph = None
+        self._sampling_cfg = cfg
+        if self.cache is not None:
+            self._sampling_params().set(counter=0, **cfg)
+
+    def _sampling_params(self):
+        """The device buffers of the sampling values, (re)made for the current cache batch and filled on creation."""
+        from . import glue
+        c = self.cache
+        if self._sampling is None or self._sampling.batch != c.batch or self._sampling.temperature.device != c.device:
+            import torch.distributed as tdist
+            rank = tdist.get_rank() if tdist.is_available() and tdist.is_initialized() else 0
+            self._sampling = glue.SamplingParams(c.batch, c.device, row_offset=rank * c.batch)   # rows of a global batch
+            self._sampling.set(counter=0, **self._sampling_cfg)
+            self._graph = None
+        return self._sampling
 
     @property
     def all_tokens(self):
@@ -701,14 +747,15 @@ class LlamaForCausalLM_KIVI(nn.Module):
     @torch.no_grad()
     def decode_step(self, input_ids=None, use_graph: bool = True):
         """One decode step for the whole batch: input_ids [B, 1] (device) -> logits [B, vocab] fp32 (device,
-        a static buffer); `next_tokens` [B] holds their argmax (and `all_tokens` every rank's, see
-        enable_token_allgather).  The step (32 x [norm, qkv, rope, fused KIVI attention, o_proj, MLP], lm_head,
+        a static buffer); `next_tokens` [B] holds their argmax, or the ids drawn with set_sampling's values (and
+        `all_tokens` every rank's, see enable_token_allgather).  The step (32 x [norm, qkv, rope, fused KIVI attention, o_proj, MLP], lm_head,
         cache advance, greedy argmax, token all-gather) is captured once in a CUDA graph and replayed."""
         assert self.cache is not None
         if self.cache.kv_len + 1 > self.cache.max_tokens:
             raise ValueError("KIVI cache capacity exceeded")
         if input_ids is not None:
             self._ids.copy_(input_ids.view(-1, 1))
+        sp = self._sampling_params() if self._sampling_cfg is not None else None   # made before a capture, never inside
         if not use_graph:
             self._step_body()
         else:
@@ -716,6 +763,7 @@ class LlamaForCausalLM_KIVI(nn.Module):
                 # warm-up on a side stream (cuBLAS workspaces, lazy module loading, NCCL channels), then capture
                 state = self.cache.state.clone()
                 pos, ids0 = self._pos.clone(), self._ids.clone()
+                ctr = sp.counter.clone() if sp is not None else None
                 s = torch.cuda.Stream()
                 s.wait_stream(torch.cuda.current_stream())
                 with torch.cuda.stream(s):
@@ -728,6 +776,8 @@ class LlamaForCausalLM_KIVI(nn.Module):
                 self.cache.state.copy_(state)
                 self._pos.copy_(pos)
                 self._ids.copy_(ids0)
+                if sp is not None:
+                    sp.counter.copy_(ctr)                                    # the warm-up step drew nothing for the caller
                 from . import _lib
                 n0 = _lib.launch_count()
                 g = torch.cuda.CUDAGraph()
@@ -745,13 +795,24 @@ class LlamaForCausalLM_KIVI(nn.Module):
 
     @torch.no_grad()
     def generate(self, input_ids=None, max_new_tokens: int | None = None, use_graph: bool = True, attention_mask=None,
-                 max_length: int | None = None, do_sample: bool = False, **unused):
-        """Greedy decoding on the fused path with the call shape of HF generate (`model.generate(**inputs,
-        max_new_tokens=n)`, example.py:60-61, mem_spd_test.py:66): returns [B, prompt + new] ids.  Sampling is outside
-        the hot path: do_sample is rejected; a padding mask must be all ones (equal-length prompts, as everywhere the
+                 max_length: int | None = None, do_sample: bool = False, temperature: float | None = None,
+                 top_k: int | None = None, top_p: float | None = None, seed: int | None = None, **unused):
+        """Decoding on the fused path with the call shape of HF generate (`model.generate(**inputs, max_new_tokens=n)`,
+        example.py:60-61, mem_spd_test.py:66): returns [B, prompt + new] ids.  do_sample=False: greedy (the model's decode
+        steps return to greedy; set_sampling's values stay for the next do_sample=True).  do_sample=True:
+        every token, the first one after the prompt included, is drawn inside the step by the sampling kernel with the
+        values given to set_sampling, overridden by any of temperature / top_k / top_p / seed given here; values never
+        given are transformers' defaults (1.0, 50, 1.0), a seed never given is drawn from torch's default generator, and
+        the draw counter restarts at every call.  A padding mask must be all ones (equal-length prompts, as everywhere the
         reference's cache keeps ONE kv_seq_len per batch, :309, :455)."""
         if do_sample:
-            raise NotImplementedError("kivi_b200.generate decodes greedily; sample from decode_step() logits instead")
+            if temperature is not None and not temperature > 0:
+                raise ValueError(f"`temperature` (={temperature}) has to be a strictly positive float when sampling")
+            cfg = dict(self._sampling_user or dict(temperature=1.0, top_k=50, top_p=1.0, seed=None))
+            given = dict(temperature=temperature, top_k=top_k, top_p=top_p, seed=seed)
+            cfg.update({k: v for k, v in given.items() if v is not None})
+        else:
+            self._activate_sampling(None)
         if attention_mask is not None and not bool(attention_mask.to(torch.bool).all()):
             raise NotImplementedError("padded prompts: use forward() with the 9-tuple cache (mask support) instead")
         B, n = input_ids.shape
@@ -763,7 +824,14 @@ class LlamaForCausalLM_KIVI(nn.Module):
             self.init_cache(B, n + max_new_tokens)
         logits = self.prefill(input_ids)
         out = [input_ids]
-        tok = logits.argmax(-1, keepdim=True)
+        if do_sample:
+            self._activate_sampling(cfg)                     # counter 0: the first draw below uses counter 1
+            sp = self._sampling_params()
+            sp.counter.add_(1)
+            from . import glue
+            tok = glue.sample(logits.contiguous(), sp, torch.empty(B, dtype=torch.long, device=logits.device)).view(B, 1)
+        else:
+            tok = logits.argmax(-1, keepdim=True)
         for _ in range(max_new_tokens - 1):
             out.append(tok)
             self.decode_step(tok, use_graph=use_graph)
