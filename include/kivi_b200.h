@@ -125,7 +125,9 @@ int kivi_unpack_dequant_lastdim_f16(const void* code, const void* scale, const v
  * int32[8] shared by all layers of a model {tk, r, tv, L, vhead, kv_len, -, -}: tk = tokens in the
  * packed K store, r = tokens in the fp16 K window, tv = tokens in the packed V store, L = tokens in
  * the fp16 V window (ring buffer starting at vhead).  All sequences of the batch have the same
- * length, as in the reference (one kv_seq_len per cache, :309, :455).
+ * length, as in the reference (one kv_seq_len per cache, :309, :455); a left-padded batch keeps
+ * that shared length and gives each sequence its first real position instead
+ * (kivi_decode_attention_padded_f16).
  * head_dim is 128 (every model the reference ships); group_size in {32,64,128};
  * residual_length % group_size == 0 (:344), residual_length in {32, 64, 128, 256}.
  * ========================================================================================== */
@@ -186,7 +188,9 @@ int64_t kivi_decode_workspace_bytes(const kivi_cache_t* cache, int max_kv_len);
  * ring and, once it holds more than R tokens, its oldest token is quantised into the V store.
  * `state` is READ ONLY here; call kivi_cache_advance once per step after the last layer.
  *   q [B, H, 128], k_new / v_new [B, Hkv, 128], out [B, H, 128]  fp16 contiguous
- *   mask: NULL or additive fp16 [B, kv_len + 1] (broadcast over heads, :364-372)
+ *   mask: NULL or additive fp16 [B, kv_len + 1] (broadcast over heads, :364-372).  Its row stride grows with
+ *   every step, so a captured graph cannot reuse one mask buffer: left padding goes through
+ *   kivi_decode_attention_padded_f16 below
  *   workspace / workspace_bytes: see kivi_decode_workspace_bytes (scaled logits rows, per-block softmax
  *   statistics, partial output records, arrival counters); no bound on the context length
  *   dbg_logits / dbg_probs: NULL or fp16 [B, H, dbg_stride] receiving s and p (tests)
@@ -204,6 +208,19 @@ int64_t kivi_decode_workspace_bytes(const kivi_cache_t* cache, int max_kv_len);
 int kivi_decode_attention_f16(const kivi_cache_t* cache, const void* q, const void* k_new, const void* v_new,
                               const void* mask, void* out, void* workspace, int64_t workspace_bytes,
                               void* dbg_logits, void* dbg_probs, int64_t dbg_stride, int max_kv_len, void* stream);
+
+/* The same step for a LEFT-PADDED batch (HF left padding + padding attention_mask, models/llama_kivi.py:364-372), with one
+ * int per sequence instead of a mask row:
+ *   seq_start: device int32 [B], required.  Positions 0 .. seq_start[b] - 1 of sequence b are padding; negative values
+ *   count as 0.  The new token (position kv_len) is never padding, so no row is ever fully masked.
+ * A padding position's scaled logit becomes what kivi_decode_attention_f16 gives for the mask value finfo(fp16).min
+ * (-65504), so probabilities and outputs are bit-identical to that call with the equivalent mask.  seq_start is read on
+ * the device by every call: a captured graph sees the values the caller copies into the same buffer before a replay.
+ * Only the packed K blocks that overlap the padding take the predicated epilogue.  The cache update is unchanged:
+ * padding tokens are quantised together with the real ones, as in the reference. */
+int kivi_decode_attention_padded_f16(const kivi_cache_t* cache, const void* q, const void* k_new, const void* v_new,
+                                     const int32_t* seq_start, void* out, void* workspace, int64_t workspace_bytes,
+                                     void* dbg_logits, void* dbg_probs, int64_t dbg_stride, int max_kv_len, void* stream);
 
 /* Test hook: the (unit, item) work split of the two decode kernels evaluated on the host (kernel 0 = q.K^T, 1 = p.V cost
  * model); a unit has n_b packed blocks, n_w window items and the new token.  out_lo: 2 * (W + 1) ints, (unit, item) of the first

@@ -35,6 +35,7 @@ def _bind():
     _lib.bind("kivi_cache_prefill_f16", i32, [P, vp, vp, i32, vp])
     _lib.bind("kivi_decode_workspace_bytes", i64, [P, i32])
     _lib.bind("kivi_decode_attention_f16", i32, [P, vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, vp])
+    _lib.bind("kivi_decode_attention_padded_f16", i32, [P, vp, vp, vp, vp, vp, vp, i64, vp, vp, i64, i32, vp])
     _lib.bind("kivi_cache_advance", i32, [P, vp])
     _lib.bind("kivi_cache_export_f16", i32, [P, i32, i32, i32, i32, i32] + [vp] * 9)
     _lib.bind("kivi_cache_import_f16", i32, [P, i32, i32, i32, i32] + [vp] * 9)
@@ -82,12 +83,36 @@ class KiviCache:
         if nws < 0:
             _lib.check(nws, "kivi_decode_workspace_bytes")
         self._ws = torch.zeros(nws, dtype=torch.uint8, device=self.device)
+        # first real position of every sequence of a left-padded batch (set_seq_start); one buffer for the cache's lifetime,
+        # so that a captured decode step reads the values copied into it later
+        self._seq_start = torch.zeros(batch, dtype=torch.int32, device=self.device)
+        self._padded = False
         # host mirror of `state` (its evolution is deterministic)
         self.tk = self.r = self.tv = self.L = self.vhead = self.kv_len = 0
 
     # ------------------------------------------------------------------ bookkeeping
     def nbytes(self) -> int:
         return self.n_layers * sum(self._bytes)
+
+    @property
+    def seq_start(self) -> torch.Tensor | None:
+        """The device int32 [B] of set_seq_start while padding is set, else None."""
+        return self._seq_start if self._padded else None
+
+    def set_seq_start(self, t):
+        """Left padding: positions 0 .. t[b] - 1 of sequence b are padding, which decode_attention masks as an additive
+        finfo(fp16).min would (kivi_decode_attention_padded_f16); negative values count as 0.  t: one int per sequence
+        (list or tensor), or None to switch padding off.  The values are copied into a buffer that never moves, so a
+        captured decode step picks up new values without a re-capture; switching padding on or off changes which kernel
+        the step launches.  prefill() and import_tuple() switch it off."""
+        if t is None:
+            self._padded = False
+            return
+        t = torch.as_tensor(t).reshape(-1)
+        if t.numel() != self.batch:
+            raise ValueError(f"seq_start needs one value per sequence ({self.batch}), got {t.numel()}")
+        self._seq_start.copy_(t.clamp(-2 ** 31, 2 ** 31 - 1).to(torch.int32))
+        self._padded = True
 
     def _mirror_prefill(self, n: int):
         R = self.residual_length
@@ -122,6 +147,7 @@ class KiviCache:
             _lib.check(_lib.lib().kivi_cache_prefill_f16(ctypes.byref(self._structs[layer]), k.data_ptr(), v.data_ptr(),
                                                          n, _lib.stream_ptr(self.device)), "kivi_cache_prefill_f16")
         self._mirror_prefill(n)
+        self._padded = False
 
     def decode_attention(self, layer: int, q: torch.Tensor, k_new: torch.Tensor, v_new: torch.Tensor,
                          mask: torch.Tensor | None = None, out: torch.Tensor | None = None,
@@ -129,7 +155,7 @@ class KiviCache:
                          ):
         """Attention of q [B,H,128] over the cache + k_new/v_new [B,Hkv,128], then the cache update for this
         layer (two launches: q.K^T + statistics, then p.V + output + update).  Call advance() once after the last
-        layer of the step."""
+        layer of the step.  While set_seq_start is in effect the left padding is masked and `mask` must be None."""
         _lib.require_cuda(q, k_new, v_new)
         assert q.shape == (self.batch, self.num_heads, self.head_dim) and q.dtype == torch.float16
         assert k_new.shape == (self.batch, self.num_kv_heads, self.head_dim) and v_new.shape == k_new.shape
@@ -139,6 +165,8 @@ class KiviCache:
         if out is None:
             out = torch.empty_like(q)
         if mask is not None:
+            if self._padded:
+                raise ValueError("decode_attention: pass either an additive mask or set_seq_start padding, not both")
             mask = mask.reshape(self.batch, -1).to(torch.float16).contiguous()
             assert mask.shape[1] == self.kv_len + 1
         stride = 0
@@ -146,14 +174,18 @@ class KiviCache:
             if d is not None:
                 assert d.dtype == torch.float16 and d.is_contiguous() and d.shape[:2] == (self.batch, self.num_heads)
                 stride = d.shape[-1]
+        if self._padded:
+            fn, name, extra = _lib.lib().kivi_decode_attention_padded_f16, "kivi_decode_attention_padded_f16", self._seq_start
+        else:
+            fn, name, extra = _lib.lib().kivi_decode_attention_f16, "kivi_decode_attention_f16", mask
         with torch.cuda.device(self.device):
-            _lib.check(_lib.lib().kivi_decode_attention_f16(
+            _lib.check(fn(
                 ctypes.byref(self._structs[layer]), q.data_ptr(), k_new.data_ptr(), v_new.data_ptr(),
-                mask.data_ptr() if mask is not None else None, out.data_ptr(),
+                extra.data_ptr() if extra is not None else None, out.data_ptr(),
                 self._ws.data_ptr(), self._ws.numel(),
                 dbg_logits.data_ptr() if dbg_logits is not None else None,
                 dbg_probs.data_ptr() if dbg_probs is not None else None, stride, self.max_tokens,
-                _lib.stream_ptr(self.device)), "kivi_decode_attention_f16")
+                _lib.stream_ptr(self.device)), name)
         return out
 
     def advance(self):
@@ -210,6 +242,7 @@ class KiviCache:
                 ctypes.byref(self._structs[layer]), tk, r, tv, L, ptr(kc), ptr(ks), ptr(km), ptr(kfull),
                 ptr(vc), ptr(vs), ptr(vm), ptr(vfull), _lib.stream_ptr(self.device)), "kivi_cache_import_f16")
         self.tk, self.r, self.tv, self.L, self.vhead, self.kv_len = tk, r, tv, L, 0, seen
+        self._padded = False
 
     def export(self, layer: int):
         """The reference's per-layer 9-tuple (models/llama_kivi.py:454-455):

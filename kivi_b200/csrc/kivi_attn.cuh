@@ -201,6 +201,7 @@ struct AttnParams {
     Workspace w;
     int stage_bytes, spw /*stages per warp*/, hchunks, n_units, nw_eff /*warps that own an sv range*/;
     int max_kv_len;                     // what the workspace rows were sized for
+    const int* seq_start;               // NULL, or [B]: positions < seq_start[b] of sequence b are left padding (qk_kernel<PAD>)
 };
 
 struct Sched {                          // per-step constants, identical for every unit
@@ -685,6 +686,13 @@ __device__ __forceinline__ __half apply_mask(__half v, const __half* mask, int64
     if (__half2float(v) < -65504.f) v = __float2half_rn(-65504.f);
     return v;
 }
+// a left-padding position: apply_mask's arithmetic with the mask value finfo(fp16).min, so that probabilities and outputs are
+// bit-identical to the additive-mask call with the equivalent mask
+__device__ __forceinline__ __half apply_pad(__half v) {
+    v = __hadd_rn(v, __float2half_rn(-65504.f));
+    if (__half2float(v) < -65504.f) v = __float2half_rn(-65504.f);
+    return v;
+}
 
 // ------------------------------------------------------------------------------------------------
 // work split: the (unit, item) sequence of the whole job -- per unit: n_b packed blocks, n_w fp16 window items, the new
@@ -830,7 +838,9 @@ __device__ __forceinline__ void qk_issue_next(Pipe& pp, Cursor& cur, const AttnP
     if (++cur.j == s.ipu) { cur.j = 0; ++cur.unit; }
 }
 
-template <int KB, int G, int GS, int CW>
+// PAD: p.seq_start is set (left-padded batch).  A compile-time flag, so that the unpadded instantiations compile to the code
+// they had without padding support (the 4-bit G = 4 kernels run 12 warps at ~160 registers and have no room to spare).
+template <int KB, int G, int GS, int CW, bool PAD>
 __global__ void __launch_bounds__(CW * 32, KIVI_MINB)
 qk_kernel(const KIVI_PARAM_QUAL AttnParams p)
 {
@@ -901,6 +911,7 @@ qk_kernel(const KIVI_PARAM_QUAL AttnParams p)
         const int u = p.hchunks == 1 ? unit : unit / p.hchunks, hc = p.hchunks == 1 ? 0 : unit % p.hchunks;
         const int b = u / c.Hkv;
         const int uq0 = u * ratio + hc * G;
+        const int pad = PAD ? max(__ldg(p.seq_start + b), 0) : 0;         // positions < pad are padding (the new token never is)
         const int j_first = j;
         const int n_here = min(left, s.ipu - j);                             // this warp's pseudo-blocks of this unit
 
@@ -955,7 +966,8 @@ qk_kernel(const KIVI_PARAM_QUAL AttnParams p)
                 float x[Slots<G, GS>::k];
                 #pragma unroll
                 for (int e = 0; e < Slots<G, GS>::k; ++e) x[e] = -INFINITY;
-                if (!slow && nvalid >= kBlockTokens) {
+                // (a block that overlaps the padding takes the predicated epilogue; the blocks after it keep the fast one)
+                if (!slow && nvalid >= kBlockTokens && (!PAD || j * kBlockTokens >= pad)) {
                     finalize<KB, G, GS>(acc, zsel, lane, 1.f, [&](int slot, int o, float v) {
                         const __half hv = scale_logit(v);
                         row[o] = hv;
@@ -966,6 +978,7 @@ qk_kernel(const KIVI_PARAM_QUAL AttnParams p)
                         if (o < nvalid) {
                             __half hv = scale_logit(v);                      // fp16 scaled (+ mask): the softmax input
                             if (p.mask) hv = apply_mask(hv, p.mask, (int64_t)b * s.T + j * kBlockTokens + o);
+                            if (PAD && j * kBlockTokens + o < pad) hv = apply_pad(hv);
                             row[o] = hv;
                             if (p.dbg_logits) p.dbg_logits[rowi * p.dbg_stride + j * kBlockTokens + o] = hv;
                             x[slot] = __half2float(hv);
@@ -1005,6 +1018,7 @@ qk_kernel(const KIVI_PARAM_QUAL AttnParams p)
                         if (t < nt) {
                             __half hv = scale_logit(e < 2 ? d0[e] : d1[e - 2]);
                             if (p.mask) hv = apply_mask(hv, p.mask, (int64_t)b * s.T + s.tk + t0 + t);
+                            if (PAD && s.tk + t0 + t < pad) hv = apply_pad(hv);   // a short prompt's padding reaches into the window
                             p.w.lg[rowi * p.w.ld + s.tk + t0 + t] = hv;
                             if (p.dbg_logits) p.dbg_logits[rowi * p.dbg_stride + s.tk + t0 + t] = hv;
                             x[e] = __half2float(hv);
@@ -1689,10 +1703,10 @@ static int launch_attention(AttnParams& p, bool overlap_prologue, cudaStream_t s
     if (tn.stages_per_warp >= 1 && tn.stages_per_warp <= p.spw) p.spw = tn.stages_per_warp;
     if (p.spw < 1) return KIVI_ERR_CAPACITY;
     const size_t smem = (size_t)kCW * p.spw * p.stage_bytes + fixed;
-    auto kqk = qk_kernel<KB, G, GS, kCW>;
+    auto kqk = p.seq_start ? qk_kernel<KB, G, GS, kCW, true> : qk_kernel<KB, G, GS, kCW, false>;
     auto ksv = sv_kernel<KB, VB, G, GS, kCW>;
-    static std::atomic<unsigned long long> optin_qk{0}, optin_sv{0};        // per kernel instantiation, one bit per device
-    rc = ensure_dynamic_smem(kqk, max_smem, di.ordinal, optin_qk); if (rc) return rc;
+    static std::atomic<unsigned long long> optin_qk{0}, optin_qk_pad{0}, optin_sv{0};   // per kernel instantiation, one bit per device
+    rc = ensure_dynamic_smem(kqk, max_smem, di.ordinal, p.seq_start ? optin_qk_pad : optin_qk); if (rc) return rc;
     rc = ensure_dynamic_smem(ksv, max_smem, di.ordinal, optin_sv); if (rc) return rc;
     const int grid = di.num_sms * ctas;
     // range owners: at least one pseudo-block each (the kernels clamp to the number of pseudo-blocks), and never more

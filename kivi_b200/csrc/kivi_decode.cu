@@ -31,9 +31,10 @@ extern "C" int64_t kivi_decode_workspace_bytes(const kivi_cache_t* cache, int ma
     return carve_workspace(c, c.B * c.Hkv * (ratio / G), G, max_kv_len, nullptr, nullptr);
 }
 
-extern "C" int kivi_decode_attention_f16(const kivi_cache_t* cache, const void* q, const void* k_new, const void* v_new,
-                                         const void* mask, void* out, void* workspace, int64_t workspace_bytes,
-                                         void* dbg_logits, void* dbg_probs, int64_t dbg_stride, int max_kv_len, void* stream)
+// the launch path of both entries: mask and seq_start are never both set
+static int decode_attention(const kivi_cache_t* cache, const void* q, const void* k_new, const void* v_new,
+                            const void* mask, const int32_t* seq_start, void* out, void* workspace, int64_t workspace_bytes,
+                            void* dbg_logits, void* dbg_probs, int64_t dbg_stride, int max_kv_len, void* stream)
 {
     AttnParams p;
     int rc = make_desc(cache, &p.c);
@@ -43,6 +44,7 @@ extern "C" int kivi_decode_attention_f16(const kivi_cache_t* cache, const void* 
     if (max_kv_len > p.c.k_cap_blocks * kBlockTokens) return KIVI_ERR_CAPACITY;
     if (reinterpret_cast<uintptr_t>(workspace) % 256 != 0) return KIVI_ERR_ALIGN;
     p.q = (const __half*)q; p.k_new = (const __half*)k_new; p.v_new = (const __half*)v_new; p.mask = (const __half*)mask;
+    p.seq_start = seq_start;
     p.out = (__half*)out; p.dbg_logits = (__half*)dbg_logits; p.dbg_probs = (__half*)dbg_probs; p.dbg_stride = dbg_stride;
     const bool overlap = (cache->flags & KIVI_CACHE_OVERLAP_PROLOGUE) != 0;   // the q.K^T launch may overlap its predecessor
     const int ratio = p.c.H / p.c.Hkv;
@@ -59,6 +61,24 @@ extern "C" int kivi_decode_attention_f16(const kivi_cache_t* cache, const void* 
     if (p.c.k_bits == 2 && p.c.v_bits == 4) return attention_k2v4(p, G, overlap, st);
     if (p.c.k_bits == 4 && p.c.v_bits == 2) return attention_k4v2(p, G, overlap, st);
     return KIVI_ERR_BITS;
+}
+
+extern "C" int kivi_decode_attention_f16(const kivi_cache_t* cache, const void* q, const void* k_new, const void* v_new,
+                                         const void* mask, void* out, void* workspace, int64_t workspace_bytes,
+                                         void* dbg_logits, void* dbg_probs, int64_t dbg_stride, int max_kv_len, void* stream)
+{
+    return decode_attention(cache, q, k_new, v_new, mask, nullptr, out, workspace, workspace_bytes, dbg_logits, dbg_probs,
+                            dbg_stride, max_kv_len, stream);
+}
+
+extern "C" int kivi_decode_attention_padded_f16(const kivi_cache_t* cache, const void* q, const void* k_new, const void* v_new,
+                                                const int32_t* seq_start, void* out, void* workspace, int64_t workspace_bytes,
+                                                void* dbg_logits, void* dbg_probs, int64_t dbg_stride, int max_kv_len,
+                                                void* stream)
+{
+    if (!seq_start) return KIVI_ERR_NULL;
+    return decode_attention(cache, q, k_new, v_new, nullptr, seq_start, out, workspace, workspace_bytes, dbg_logits, dbg_probs,
+                            dbg_stride, max_kv_len, stream);
 }
 
 // Test hook (tests/test_ranges_cpu.py): the work split of the decode kernels, evaluated on the host.  kernel 0 = q.K^T costs,

@@ -330,6 +330,30 @@ def _additive_mask(attention_mask, q_len: int, total: int, dtype, device):
     return torch.zeros(keep.shape, dtype=dtype, device=device).masked_fill(~keep, torch.finfo(dtype).min)
 
 
+def _left_padding(attention_mask):
+    """HF padding mask [B, n] (1 = real token) -> (pad [B], positions [B, n]), both int64 on the mask's device, or None when
+    nothing is padded.  pad[b] counts the leading zeros of row b; positions are those of prepare_inputs_for_generation
+    (cumsum - 1, padding at 1).  The fused cache path supports LEFT padding only: the zeros of every row must form a prefix.
+    Right padding or holes raise NotImplementedError, a row without a real token ValueError."""
+    if attention_mask is None:
+        return None
+    if attention_mask.dim() != 2:
+        raise NotImplementedError("the fused cache path takes a 2-D HF padding mask [batch, tokens] with left padding")
+    keep = attention_mask.to(torch.bool)
+    if bool(keep.all()):
+        return None
+    if not bool(keep.any(-1).all()):
+        raise ValueError("attention_mask has a row without any real token")
+    m = keep.long()
+    if not bool((m[:, 1:] >= m[:, :-1]).all()):
+        raise NotImplementedError("the fused cache path supports left padding only (the zeros of every attention_mask row "
+                                  "must form a prefix); right padding and holes are not supported")
+    pad = m.shape[1] - m.sum(-1)
+    positions = m.cumsum(-1) - 1
+    positions.masked_fill_(m == 0, 1)
+    return pad, positions
+
+
 class LlamaForCausalLM_KIVI(nn.Module):
     """models/llama_kivi.py:785.  `forward` keeps the reference's contract (HF argument names, per-layer 9-tuples as
     past_key_values, fp32 logits, `prepare_inputs_for_generation`, `_reorder_cache`); `decode_step` / `generate` use
@@ -344,6 +368,7 @@ class LlamaForCausalLM_KIVI(nn.Module):
         self._rope = None
         self.cache: KiviCache | None = None
         self._graph = None
+        self._graph_padded = False          # whether the captured step launches the padded attention (cache.seq_start set)
         self._fast = None
         self._dist_tokens = None            # [world * B] ids gathered inside the step (greedy sampling, world > 1)
         self._dist_in_graph = True
@@ -565,20 +590,34 @@ class LlamaForCausalLM_KIVI(nn.Module):
         return self.cache
 
     @torch.no_grad()
-    def prefill(self, input_ids):
-        """Run the prompt, fill the cache (models/llama_kivi.py:401-452), return last-position logits."""
+    def prefill(self, input_ids, attention_mask=None):
+        """Run the prompt, fill the cache (models/llama_kivi.py:401-452), return last-position logits.
+        attention_mask: None, or an HF padding mask [B, n] with LEFT padding (the zeros of every row form a prefix).  The
+        prompt then runs with HF's positions and padding mask, and the decode steps mask the padding of every sequence
+        (KiviCache.set_seq_start) and continue its positions from its number of real tokens."""
         assert self.cache is not None, "call init_cache() first"
         B, n = input_ids.shape
-        positions = torch.arange(n, device=input_ids.device).unsqueeze(0).expand(B, -1)
+        if attention_mask is not None and tuple(attention_mask.shape) != (B, n):
+            raise ValueError(f"attention_mask of shape {tuple(attention_mask.shape)} for input_ids of shape {(B, n)}")
+        padding = _left_padding(attention_mask)
         pasts = [(self.cache, i) for i in range(len(self.model.layers))]
-        h, _ = self._run_layers(input_ids, positions, pasts)
-        self._pos.fill_(n)
+        if padding is None:
+            positions = torch.arange(n, device=input_ids.device).unsqueeze(0).expand(B, -1)
+            h, _ = self._run_layers(input_ids, positions, pasts)
+            self._pos.fill_(n)
+        else:
+            pad, positions = padding
+            mask = _additive_mask(attention_mask, n, n, self.lm_head.weight.dtype, input_ids.device)
+            h, _ = self._run_layers(input_ids, positions.to(input_ids.device), pasts, mask)
+            self._pos.copy_((n - pad).view(B, 1))
+            self.cache.set_seq_start(pad)                    # after the layers: KiviCache.prefill switches padding off
         return self.lm_head(h[:, -1]).float()
 
     @torch.no_grad()
-    def prefill_synthetic(self, n: int, seed: int = 0):
+    def prefill_synthetic(self, n: int, seed: int = 0, seq_start=None):
         """Fill every layer's cache with n random K/V tokens (benchmarks: the prompt's attention itself is
-        off the decode hot path; the cache contents are produced by the real prefill pack kernels)."""
+        off the decode hot path; the cache contents are produced by the real prefill pack kernels).
+        seq_start: None, or one int per sequence: its first real position (left padding, as prefill with a mask sets it)."""
         assert self.cache is not None
         c = self.cache
         gen = torch.Generator(device=c.device).manual_seed(seed)
@@ -587,6 +626,9 @@ class LlamaForCausalLM_KIVI(nn.Module):
             v = torch.randn((c.batch, c.num_kv_heads, n, c.head_dim), generator=gen, device=c.device, dtype=torch.float16)
             c.prefill(l, k, v)
         self._pos.fill_(n)
+        if seq_start is not None:
+            c.set_seq_start(seq_start)
+            self._pos.copy_((n - c.seq_start.long().clamp(0, n)).view(c.batch, 1))
 
     def _step_body(self):
         if self._fast_ok():
@@ -756,6 +798,9 @@ class LlamaForCausalLM_KIVI(nn.Module):
         if input_ids is not None:
             self._ids.copy_(input_ids.view(-1, 1))
         sp = self._sampling_params() if self._sampling_cfg is not None else None   # made before a capture, never inside
+        padded = self.cache.seq_start is not None
+        if self._graph is not None and self._graph_padded != padded:
+            self._graph = None                               # the captured step launches the other attention entry
         if not use_graph:
             self._step_body()
         else:
@@ -785,7 +830,7 @@ class LlamaForCausalLM_KIVI(nn.Module):
                     self._step_body()
                 self.launches_per_step = _lib.launch_count() - n0            # libkivi_b200 launches replayed by every step
                 # capture does not execute: state is still the pre-step state
-                self._graph = g
+                self._graph, self._graph_padded = g, padded
             self._graph.replay()
         if self._dist_tokens is not None and not self._dist_in_graph:
             from . import dist as kdist
@@ -803,8 +848,9 @@ class LlamaForCausalLM_KIVI(nn.Module):
         every token, the first one after the prompt included, is drawn inside the step by the sampling kernel with the
         values given to set_sampling, overridden by any of temperature / top_k / top_p / seed given here; values never
         given are transformers' defaults (1.0, 50, 1.0), a seed never given is drawn from torch's default generator, and
-        the draw counter restarts at every call.  A padding mask must be all ones (equal-length prompts, as everywhere the
-        reference's cache keeps ONE kv_seq_len per batch, :309, :455)."""
+        the draw counter restarts at every call.  attention_mask: an HF padding mask with LEFT padding (prefill): the batch
+        keeps one kv_seq_len, as the reference's cache does (:309, :455), and every sequence's padding is masked in every
+        step; the padding stays on the left of the returned ids, as HF returns them."""
         if do_sample:
             if temperature is not None and not temperature > 0:
                 raise ValueError(f"`temperature` (={temperature}) has to be a strictly positive float when sampling")
@@ -813,16 +859,15 @@ class LlamaForCausalLM_KIVI(nn.Module):
             cfg.update({k: v for k, v in given.items() if v is not None})
         else:
             self._activate_sampling(None)
-        if attention_mask is not None and not bool(attention_mask.to(torch.bool).all()):
-            raise NotImplementedError("padded prompts: use forward() with the 9-tuple cache (mask support) instead")
         B, n = input_ids.shape
+        _left_padding(attention_mask)                        # a mask the fused path cannot run raises before any work
         if max_new_tokens is None:
             if max_length is None:
                 raise ValueError("generate() needs max_new_tokens or max_length")
             max_new_tokens = max_length - n
         if self.cache is None or self.cache.batch != B or self.cache.max_tokens < n + max_new_tokens:
             self.init_cache(B, n + max_new_tokens)
-        logits = self.prefill(input_ids)
+        logits = self.prefill(input_ids, attention_mask)
         out = [input_ids]
         if do_sample:
             self._activate_sampling(cfg)                     # counter 0: the first draw below uses counter 1
